@@ -2,7 +2,7 @@
 """bench.py — BASELINE metric: 3D patches/sec (128^3) of the Retina U-Net train step (lidc_exp config, synthetic 1-channel patches,
 batch 2 per GPU), on N B200s of one node.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--patch 128 128 128] [--batch 2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--patch 128 128 128] [--batch 2] [--dump-outputs DIR]
 
 A step = train_forward (H2D of the batch, FPN + heads on the tcgen05/SIMT conv kernels, on-device anchor matching, losses, batched NMS,
 results D2H) + backward + (N > 1: one NCCL all-reduce of the flat fp32 gradient buffer) + Adam.
@@ -93,15 +93,11 @@ def run_reference(args):
     torch.set_num_threads(cores)
     patch = tuple(args.patch)
     cf = make_cf('retina_unet', 3, patch)
-    # same config as the GPU arm: batch, warm-up and step count as requested; only if W + K steps would exceed the time box (a CPU step of
-    # 2 x 128^3 patches takes ~14 s) the number of TIMED steps shrinks — never the batch or the warm-up
+    # same config as the GPU arm: batch, warm-up and timed step count exactly as requested (a CPU step of 2 x 128^3 patches takes ~14 s)
     b = args.batch
     batch = synthetic_batch(cf, b, seed=0)
-    t_first, used = cpu_step.time_cpu_steps(cf, batch, steps=1, warmup=0, threads=cores)
-    budget = float(os.environ.get("MDT_REF_BUDGET_S", "540"))
     warm = args.warmup
-    steps = max(1, min(args.steps, int(budget / max(t_first[0], 1e-3)) - warm - 1))
-    times, used = cpu_step.time_cpu_steps(cf, batch, steps=steps, warmup=max(warm - 1, 0), threads=cores)   # the probe step above was warm-up 1
+    times, used = cpu_step.time_cpu_steps(cf, batch, steps=args.steps, warmup=warm, threads=cores)
     ms = 1e3 * sum(times) / len(times)
     val = b / (ms / 1e3)
     sample = "%d full train step(s) of %d patch(es) %s (forward+detections+matching+losses+backward+Adam), fp32, torch CPU" % (len(times), b, "x".join(map(str, patch)))
@@ -162,6 +158,31 @@ def make_roofline(step_flops, conv_ms, n_conv_calls, ms_step, dom, peak_tf, peak
     roof["peak_source"] = src
     roof["all_conv_launches"] = agg
     return roof
+
+
+DUMP_MAX_ELEMS = 1 << 22    # per array (16 MB in float32): segmentation + parameters + the small arrays stay under 64 MB in all
+
+
+def step_outputs(res, net, dim):
+    """What a caller of one train step receives, as float32 / float64 numpy arrays: the loss, the monitor values, the detections (rows
+    [batch index, 2 * dim box coordinates, class id, score]), the segmentation and the parameters after the optimizer step (flattened in
+    net.parameters() order).  An array of more than DUMP_MAX_ELEMS values is replaced by a fixed, seeded sample of its flattened values.
+    Copies everything: train_forward's host buffers are reused by the next step."""
+    import numpy as np
+    import torch
+    out = {"loss": np.array([float(res['torch_loss'])], dtype=np.float64)}
+    for k, v in res['monitor_values'].items():
+        out["monitor_" + k] = np.array([float(v)], dtype=np.float64)
+    dets = [[b] + [float(c) for c in bx['box_coords']] + [float(bx['box_pred_class_id']), float(bx['box_score'])]
+            for b, boxes in enumerate(res['boxes']) for bx in boxes if bx['box_type'] == 'det']
+    out["detections"] = np.array(dets, dtype=np.float64).reshape(len(dets), 2 * dim + 3)
+    out["seg_preds"] = np.asarray(res['seg_preds'], dtype=np.float32).copy()
+    out["parameters"] = torch.cat([p.detach().reshape(-1).float() for p in net.parameters()]).cpu().numpy()
+    for k, a in out.items():
+        if a.size > DUMP_MAX_ELEMS:
+            ix = np.sort(np.random.RandomState(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))
+            out[k] = a.reshape(-1)[ix]
+    return out
 
 
 def capture_logits_graph(net, batch, lib, eager_logits, reducer):
@@ -232,7 +253,14 @@ def main():
                          "(53.9 vs 51.8 ms: the conv part is not launch-bound, the replay adds node-to-node latency), hence opt-in")
     ap.add_argument("--model", default="retina_unet", choices=["retina_unet", "mrcnn"],
                     help="retina_unet = BASELINE configs[1] (the metric's config); mrcnn = configs[2]: 3D Mask R-CNN, 512 proposals, RoIAlign 7x7x3")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (bench.step_outputs) to DIR/<name>.npy; the inputs "
+                         "are seeded, so two builds can be compared output for output.  Inside the tree, bench_outputs/ is ignored by git")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -299,11 +327,13 @@ def main():
         torch.cuda.synchronize()
 
     def timed(batches, n):
+        """(ms for n steps, the last step's result)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for i in range(n):
+        for i in range(n - 1):
             step(batches[i % len(batches)])
+        res = step(batches[(n - 1) % len(batches)])
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -311,7 +341,7 @@ def main():
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms
+        return ms, res
 
     for i in range(max(args.warmup, 1)):
         step(dev_batches[i % 2])
@@ -338,8 +368,10 @@ def main():
     # --- kernel-resident throughput (inputs already in HBM), uninstrumented
     launches0 = lib.mdt_launch_count()
     torch.cuda.profiler.start()     # no-op unless run under `ncu --profile-from-start off`: the launch list then covers exactly the timed steps
-    ms_dev = timed(dev_batches, args.steps)
+    ms_dev, last = timed(dev_batches, args.steps)
     torch.cuda.profiler.stop()
+    dumped = step_outputs(last, net, cf.dim) if args.dump_outputs and rank == 0 else None
+    del last
     launches = lib.mdt_launch_count() - launches0 + graph["kernels_per_step"] * args.steps   # eager launches + kernel nodes replayed from the graphs
     # --- separate instrumented pass: every conv call bracketed by CUDA events on the launching stream (roofline object only)
     conv_ms = None
@@ -374,7 +406,7 @@ def main():
         for i in range(min(args.steps, 4)):                   # keep the ranks in step (the all-reduce is collective)
             step(dev_batches[i % 2])
     # --- end to end through the public API with host buffers
-    ms_e2e = timed(host_batches, args.steps)
+    ms_e2e, _ = timed(host_batches, args.steps)
     if rank == 0:
         sampler.stop_flag.set()
         sampler.join(timeout=3)
@@ -423,6 +455,10 @@ def main():
         line["cpu_baseline"] = {"value": args.batch / times[0], "unit": "patches/s", "cores": used, "host_cpus": os.cpu_count(), "cpu_model": cpu_model(),
                                 "kind": "port",
                                 "sample": "1 full train step of %d patches %s on the host cores (oracle/cpu_step.py: torch CPU fp32 convs, numpy fp64 matching, C NMS)" % (args.batch, "x".join(map(str, patch)))}
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, k + ".npy"), a)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

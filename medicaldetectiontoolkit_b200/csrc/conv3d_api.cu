@@ -18,7 +18,8 @@ static bool pw_backward(const mdt_conv3d_desc *c, const ConvGeom &g, bool need_d
 }
 static size_t simt_ws(const ConvGeom &g, int pass, int algo) {
     if (algo == 4) return conv_pw_workspace_bytes(g, pass);
-    return pass == 2 ? 0 : sizeof(float) * (size_t)g.cout * g.cin * g.kd * g.kh * g.kw;
+    if (pass == 2) return conv_stem_supported(g, 2) ? conv_stem_wgrad_workspace_bytes(g) : conv_simt_wgrad_workspace_bytes(g);
+    return sizeof(float) * (size_t)g.cout * g.cin * g.kd * g.kh * g.kw;
 }
 }  // namespace mdt
 
@@ -80,8 +81,8 @@ int mdt_conv3d_wgrad(const mdt_conv3d_desc *c, const float *x, const float *dy, 
     if (algo == 0) return MDT_EUNSUPPORTED;
     if (algo == 2) return mdt::conv_tc_wgrad(g, x, dy, dw, db, c->precision, ws, ws_bytes, mdt::as_stream(stream));
     if (algo == 4) return mdt::conv_pw_wgrad(g, x, dy, nullptr, dw, db, ws, ws_bytes, mdt::as_stream(stream));
-    if (mdt::conv_stem_supported(g, 2)) return mdt::conv_stem_wgrad(g, x, dy, dw, db, mdt::as_stream(stream));
-    return mdt::conv_simt_wgrad(g, x, dy, dw, db, mdt::as_stream(stream));
+    if (mdt::conv_stem_supported(g, 2)) return mdt::conv_stem_wgrad(g, x, dy, dw, db, ws, ws_bytes, mdt::as_stream(stream));
+    return mdt::conv_simt_wgrad(g, x, dy, dw, db, ws, ws_bytes, mdt::as_stream(stream));
 }
 
 /* fused backward: 1 if the tcgen05 fused path (one pass over dy shared by dgrad + wgrad, ReLU mask and bias gradient folded in) applies */

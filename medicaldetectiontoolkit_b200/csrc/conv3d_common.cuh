@@ -26,13 +26,19 @@ inline bool make_geom(const mdt_conv3d_desc *c, ConvGeom &g) {
 int conv_simt_fprop(const ConvGeom &g, const float *x, const float *w, const float *bias, const float *residual, float *y, int relu, void *ws,
                     cudaStream_t st);
 int conv_simt_dgrad(const ConvGeom &g, const float *dy, const float *w, float *dx, void *ws, cudaStream_t st);
-int conv_simt_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, cudaStream_t st);
-int conv_bias_grad(const ConvGeom &g, const float *dy, float *db, cudaStream_t st);
+int conv_simt_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, void *ws, size_t ws_bytes, cudaStream_t st);
+size_t conv_simt_wgrad_workspace_bytes(const ConvGeom &g);
+int conv_bias_grad(const ConvGeom &g, const float *dy, float *db, void *ws, size_t ws_bytes, cudaStream_t st);
+size_t conv_bias_grad_workspace_bytes(const ConvGeom &g);
+// out[e] = sum over b = 0 .. nb-1 of partial[b * n + e], always in the same order: the per-block partial sums of a reduction are combined
+// here instead of with float atomics, so gradients are bitwise reproducible from run to run
+int reduce_partials(const float *partial, int nb, long long n, float *out, cudaStream_t st);
 
 // direct stem kernels, Cin <= 4 (conv3d_stem.cu)
 bool conv_stem_supported(const ConvGeom &g, int pass);
 int conv_stem_fprop(const ConvGeom &g, const float *x, const float *w, const float *bias, float *y, int relu, cudaStream_t st);
-int conv_stem_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, cudaStream_t st);
+int conv_stem_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, void *ws, size_t ws_bytes, cudaStream_t st);
+size_t conv_stem_wgrad_workspace_bytes(const ConvGeom &g);
 
 // pointwise 1x1x1 stride-1 fp32 streaming kernels (conv3d_pw.cu)
 bool conv_pw_supported(const ConvGeom &g, int pass);

@@ -136,8 +136,9 @@ __global__ void __launch_bounds__(256) conv_igemm_simt(ConvGeom g, const float *
 // wgrad: grid (tap, m-split, ci-tile * co-tile).  Tile 32 (ci) x 64 (co), BKW voxels per step, 256 threads each 2 x 4.
 constexpr int WCI = 32, WCO = 64, BKW = 32;
 
+// partial[split][co][ci][tap]: the weight gradient of the rows of one split (blockIdx.y); reduce_partials sums the splits
 __global__ void __launch_bounds__(256) conv_wgrad_simt(ConvGeom g, const float *__restrict__ x, const float *__restrict__ dy,
-                                                      float *__restrict__ dw, long long rows_per_split) {
+                                                      float *__restrict__ partial, long long rows_per_split) {
     const int taps = g.kd * g.kh * g.kw;
     const int t = blockIdx.x;
     const int kw_ = t % g.kw, kh_ = (t / g.kw) % g.kh, kd_ = t / (g.kw * g.kh);
@@ -196,14 +197,14 @@ __global__ void __launch_bounds__(256) conv_wgrad_simt(ConvGeom g, const float *
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int ci = ci0 + tci + i, co = co0 + tco + j;
-            if (ci < g.cin && co < g.cout && acc[i][j] != 0.f) atomicAdd(dw + ((size_t)co * g.cin + ci) * taps + t, acc[i][j]);
+            if (ci < g.cin && co < g.cout) partial[(size_t)blockIdx.y * g.cout * g.cin * taps + ((size_t)co * g.cin + ci) * taps + t] = acc[i][j];
         }
 }
 
 // db[co] = sum_m dy[m, co].  dy is read as a FLAT array: the block walks it in strides of S = (256 / cout) * cout elements, so thread t always
 // owns channel t % cout and a warp's loads are 32 consecutive floats (fully coalesced, no idle channel lanes); 4 independent accumulators
-// keep 4 loads in flight per thread.  Shared-memory tree over the row lanes, one atomicAdd per channel per block.
-__global__ void __launch_bounds__(256) bias_grad_kernel(const float *__restrict__ dy, float *__restrict__ db, long long M, int cout,
+// keep 4 loads in flight per thread.  Shared-memory tree over the row lanes; partial[block][co] is the sum of the block's rows.
+__global__ void __launch_bounds__(256) bias_grad_kernel(const float *__restrict__ dy, float *__restrict__ partial, long long M, int cout,
                                                        long long rows_per_block) {
     __shared__ float red[256];
     const long long m0 = (long long)blockIdx.x * rows_per_block, m1 = min(M, m0 + rows_per_block);
@@ -223,13 +224,13 @@ __global__ void __launch_bounds__(256) bias_grad_kernel(const float *__restrict_
         if ((int)threadIdx.x < cout) {
             float t = 0.f;
             for (int r = 0; r < nrl; ++r) t += red[r * cout + threadIdx.x];
-            atomicAdd(db + threadIdx.x, t);
+            partial[(long long)blockIdx.x * cout + threadIdx.x] = t;
         }
     } else {
         for (int c = threadIdx.x; c < cout; c += 256) {
             float s = 0.f;
             for (long long m = m0; m < m1; ++m) s += __ldg(dy + m * cout + c);
-            atomicAdd(db + c, s);
+            partial[(long long)blockIdx.x * cout + c] = s;
         }
     }
 }
@@ -259,39 +260,79 @@ int conv_simt_dgrad(const ConvGeom &g, const float *dy, const float *w, float *d
     return launch_status();
 }
 
-int conv_bias_grad(const ConvGeom &g, const float *dy, float *db, cudaStream_t st) {
-    const long long M = (long long)g.n * g.od * g.oh * g.ow;
-    cudaError_t e = cudaMemsetAsync(db, 0, sizeof(float) * g.cout, st);
-    if (e != cudaSuccess) return (int)e;
-    // rows per block: 1024 for the full-resolution maps (one atomic per channel and block), down to 32 for the small deep maps — the wide
-    // (cout > 256) path walks its rows serially per thread and took 113-146 us on 1-4 blocks for 1-5 MB tensors (profiles/r02_ncu_launches.csv)
-    long long blocks_ll = ceil_div<long long>(M, g.cout > 256 ? 32 : (M >= 262144 ? 1024 : 128));
-    if (blocks_ll > (long long)num_sms() * 8) blocks_ll = (long long)num_sms() * 8;
-    const int blocks = (int)blocks_ll;
-    bias_grad_kernel<<<blocks, 256, 0, st>>>(dy, db, M, g.cout, ceil_div<long long>(M, blocks));
+__global__ void __launch_bounds__(256) reduce_partials_kernel(const float *__restrict__ partial, int nb, long long n, float *__restrict__ out) {
+    // one warp per output element: lane l sums partials l, l + 32, ... in order, then a fixed butterfly combines the 32 lane sums
+    const long long e = ((long long)blockIdx.x * blockDim.x + threadIdx.x) / 32;
+    const int lane = threadIdx.x & 31;
+    if (e >= n) return;   // warp-uniform
+    float s = 0.f;
+    for (int b = lane; b < nb; b += 32) s += __ldg(partial + (long long)b * n + e);
+#pragma unroll
+    for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) out[e] = s;
+}
+
+int reduce_partials(const float *partial, int nb, long long n, float *out, cudaStream_t st) {
+    reduce_partials_kernel<<<(unsigned)ceil_div<long long>(n * 32, 256), 256, 0, st>>>(partial, nb, n, out);
     return launch_status();
 }
 
-int conv_simt_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, cudaStream_t st) {
+static int bias_grad_blocks(const ConvGeom &g) {
+    const long long M = (long long)g.n * g.od * g.oh * g.ow;
+    // rows per block: 1024 for the full-resolution maps, down to 32 for the small deep maps — the wide (cout > 256) path walks its rows
+    // serially per thread and took 113-146 us on 1-4 blocks for 1-5 MB tensors (profiles/r02_ncu_launches.csv)
+    long long blocks = ceil_div<long long>(M, g.cout > 256 ? 32 : (M >= 262144 ? 1024 : 128));
+    if (blocks > (long long)num_sms() * 8) blocks = (long long)num_sms() * 8;
+    return (int)blocks;
+}
+
+size_t conv_bias_grad_workspace_bytes(const ConvGeom &g) { return sizeof(float) * (size_t)bias_grad_blocks(g) * g.cout; }
+
+int conv_bias_grad(const ConvGeom &g, const float *dy, float *db, void *ws, size_t ws_bytes, cudaStream_t st) {
+    if (!ws || ws_bytes < conv_bias_grad_workspace_bytes(g)) return MDT_EWORKSPACE;
+    const long long M = (long long)g.n * g.od * g.oh * g.ow;
+    const int blocks = bias_grad_blocks(g);
+    float *partial = reinterpret_cast<float *>(ws);
+    bias_grad_kernel<<<blocks, 256, 0, st>>>(dy, partial, M, g.cout, ceil_div<long long>(M, blocks));
+    const int rc = launch_status();
+    if (rc) return rc;
+    return reduce_partials(partial, blocks, g.cout, db, st);
+}
+
+// rows of M per split (a multiple of BKW) and the number of splits of the SIMT weight gradient
+static void simt_wgrad_splits(const ConvGeom &g, long long &splits, long long &rows) {
     const int taps = g.kd * g.kh * g.kw;
-    cudaError_t e = cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)g.cout * g.cin * taps, st);
-    if (e != cudaSuccess) return (int)e;
     const long long M = (long long)g.n * g.od * g.oh * g.ow;
     const int tiles = ceil_div(g.cin, WCI) * ceil_div(g.cout, WCO);
     // enough CTAs to fill the machine a few times over, but at least 4 * BKW rows each
-    long long want = ceil_div<long long>((long long)num_sms() * 16, (long long)taps * tiles);
-    long long splits = want;
+    splits = ceil_div<long long>((long long)num_sms() * 16, (long long)taps * tiles);
     if (splits > ceil_div<long long>(M, 4 * BKW)) splits = ceil_div<long long>(M, 4 * BKW);
     if (splits < 1) splits = 1;
     if (splits > 65535) splits = 65535;
-    long long rows = ceil_div<long long>(M, splits);
-    rows = ceil_div<long long>(rows, BKW) * BKW;
+    rows = ceil_div<long long>(ceil_div<long long>(M, splits), BKW) * BKW;
     splits = ceil_div<long long>(M, rows);
+}
+
+size_t conv_simt_wgrad_workspace_bytes(const ConvGeom &g) {
+    long long splits, rows;
+    simt_wgrad_splits(g, splits, rows);
+    const size_t w = sizeof(float) * (size_t)splits * g.cout * g.cin * g.kd * g.kh * g.kw, b = conv_bias_grad_workspace_bytes(g);
+    return w > b ? w : b;
+}
+
+int conv_simt_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, void *ws, size_t ws_bytes, cudaStream_t st) {
+    if (!ws || ws_bytes < conv_simt_wgrad_workspace_bytes(g)) return MDT_EWORKSPACE;
+    const int taps = g.kd * g.kh * g.kw;
+    const int tiles = ceil_div(g.cin, WCI) * ceil_div(g.cout, WCO);
+    long long splits, rows;
+    simt_wgrad_splits(g, splits, rows);
+    float *partial = reinterpret_cast<float *>(ws);
     dim3 grid(taps, (unsigned)splits, tiles);
-    conv_wgrad_simt<<<grid, 256, 0, st>>>(g, x, dy, dw, rows);
+    conv_wgrad_simt<<<grid, 256, 0, st>>>(g, x, dy, partial, rows);
     int rc = launch_status();
     if (rc) return rc;
-    if (db) return conv_bias_grad(g, dy, db, st);
+    if ((rc = reduce_partials(partial, (int)splits, (long long)g.cout * g.cin * taps, dw, st))) return rc;
+    if (db) return conv_bias_grad(g, dy, db, ws, ws_bytes, st);   // reuses the workspace after the reduction (same stream)
     return MDT_OK;
 }
 

@@ -73,8 +73,8 @@ __global__ void __launch_bounds__(256) stem_fprop_kernel(ConvGeom g, const float
     }
 }
 
-// one block per (n, od, oh) output line; requires sw == 1
-__global__ void __launch_bounds__(256) stem_wgrad_kernel(ConvGeom g, const float *__restrict__ x, const float *__restrict__ dy, float *__restrict__ dw,
+// one block per (n, od, oh) output line; requires sw == 1.  partial[block][co][ci][tap]: the weight gradient of the block's lines
+__global__ void __launch_bounds__(256) stem_wgrad_kernel(ConvGeom g, const float *__restrict__ x, const float *__restrict__ dy, float *__restrict__ partial,
                                                         long long lines_per_block) {
     extern __shared__ float smem[];
     const int T = g.kd * g.kh * g.kw;
@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(256) stem_wgrad_kernel(ConvGeom g, const float
 #pragma unroll
     for (int q = 0; q < kPer; ++q) {
         const int pidx = threadIdx.x + q * 256;
-        if (pidx < npairs && acc[q] != 0.f) atomicAdd(dw + pidx, acc[q]);   // dw layout [co][ci][tap] == pidx order
+        if (pidx < npairs) partial[(long long)blockIdx.x * npairs + pidx] = acc[q];   // dw layout [co][ci][tap] == pidx order
     }
 }
 
@@ -195,9 +195,10 @@ __global__ void __launch_bounds__(256) stem_fprop_c1k3_kernel(ConvGeom g, const 
 
 // wgrad: dw[co][tap] = sum_v dy[v][co] * x[v + tap].  A block works on kStemWgLines output lines at once; within a line a thread owns a
 // 3 (co) x 3 (kw) register tile of one (kd, kh) pair and slides along the line: per voxel 3 dy loads + 1 new x value feed 9 FMAs (the generic
-// kernel: 2 loads per FMA).  Partials are kept in registers over all lines of the block and combined with one atomicAdd per element per block.
+// kernel: 2 loads per FMA).  Partials are kept in registers over all lines of the block; the kStemWgLines threads of an element are summed
+// in shared memory in line order and written to partial[block][co][tap].
 constexpr int kStemWgLines = 4, kStemWgCoT = 3;
-__global__ void __launch_bounds__(256) stem_wgrad_c1k3_kernel(ConvGeom g, const float *__restrict__ x, const float *__restrict__ dy, float *__restrict__ dw,
+__global__ void __launch_bounds__(256) stem_wgrad_c1k3_kernel(ConvGeom g, const float *__restrict__ x, const float *__restrict__ dy, float *__restrict__ partial,
                                                              long long groups_per_block) {
     extern __shared__ float smem[];
     const int W = g.w, XW = W + 2;
@@ -252,14 +253,26 @@ __global__ void __launch_bounds__(256) stem_wgrad_c1k3_kernel(ConvGeom g, const 
             }
         }
     }
+    __syncthreads();
+    float *s_red = smem;                                     // [line][per_line][kStemWgCoT * 3]
     if (active) {
+#pragma unroll
+        for (int a = 0; a < kStemWgCoT; ++a)
+#pragma unroll
+            for (int b = 0; b < 3; ++b) s_red[((size_t)lt * per_line + li) * (kStemWgCoT * 3) + a * 3 + b] = acc[a][b];
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < per_line) {
 #pragma unroll
         for (int a = 0; a < kStemWgCoT; ++a) {
             const int co = cg * kStemWgCoT + a;
             if (co >= g.cout) continue;
 #pragma unroll
-            for (int b = 0; b < 3; ++b)
-                if (acc[a][b] != 0.f) atomicAdd(dw + (size_t)co * 27 + kdh * 3 + b, acc[a][b]);   // dw [co][1][kd][kh][kw]
+            for (int b = 0; b < 3; ++b) {
+                float t = 0.f;
+                for (int l = 0; l < kStemWgLines; ++l) t += s_red[((size_t)l * per_line + li) * (kStemWgCoT * 3) + a * 3 + b];
+                partial[(long long)blockIdx.x * g.cout * 27 + (size_t)co * 27 + kdh * 3 + b] = t;   // dw [co][1][kd][kh][kw]
+            }
         }
     }
 }
@@ -292,36 +305,58 @@ int conv_stem_fprop(const ConvGeom &g, const float *x, const float *w, const flo
     return launch_status();
 }
 
-int conv_stem_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, cudaStream_t st) {
-    const int T = g.kd * g.kh * g.kw;
-    cudaError_t e = cudaMemsetAsync(dw, 0, sizeof(float) * (size_t)g.cout * g.cin * T, st);
-    if (e != cudaSuccess) return (int)e;
+// launch shape of the weight gradient: the c1k3 kernel (c1k3 = true) or the generic one, its block count and dynamic shared memory
+struct StemWgradPlan {
+    bool c1k3;
+    long long blocks, per_block;
+    size_t smem;
+};
+
+static StemWgradPlan stem_wgrad_plan(const ConvGeom &g) {
+    StemWgradPlan p;
     const long long nlines = (long long)g.n * g.od * g.oh;
-    {
-        const int per_line = ceil_div(g.cout, kStemWgCoT) * 9;
-        const size_t smem3 = (size_t)kStemWgLines * ((size_t)g.w * g.cout + 9 * (g.w + 2)) * sizeof(float);
-        if (stem_c1k3(g) && per_line * kStemWgLines <= 256 && smem3 <= 96 * 1024 && !getenv("MDT_STEM_GENERIC")) {
-            const long long ngroups = ceil_div<long long>(nlines, kStemWgLines);
-            long long blocks3 = (long long)num_sms() * 4;
-            if (blocks3 > ngroups) blocks3 = ngroups;
-            static bool attr3[kMaxDevices] = {};
-            if (!ensure_smem_attr(stem_wgrad_c1k3_kernel, 96 * 1024, attr3)) return MDT_EDRIVER;
-            stem_wgrad_c1k3_kernel<<<(unsigned)blocks3, 256, smem3, st>>>(g, x, dy, dw, ceil_div<long long>(ngroups, blocks3));
-            int rc3 = launch_status();
-            if (rc3) return rc3;
-            if (db) return conv_bias_grad(g, dy, db, st);
-            return MDT_OK;
-        }
+    const int per_line = ceil_div(g.cout, kStemWgCoT) * 9;
+    const size_t stage3 = (size_t)kStemWgLines * ((size_t)g.w * g.cout + 9 * (g.w + 2)) * sizeof(float);
+    const size_t red3 = (size_t)kStemWgLines * per_line * kStemWgCoT * 3 * sizeof(float);   // the final per-block combination reuses the buffer
+    p.smem = stage3 > red3 ? stage3 : red3;
+    p.c1k3 = stem_c1k3(g) && per_line * kStemWgLines <= 256 && p.smem <= 96 * 1024 && !getenv("MDT_STEM_GENERIC");
+    if (p.c1k3) {
+        const long long ngroups = ceil_div<long long>(nlines, kStemWgLines);
+        p.blocks = (long long)num_sms() * 4;
+        if (p.blocks > ngroups) p.blocks = ngroups;
+        p.per_block = ceil_div<long long>(ngroups, p.blocks);
+    } else {
+        p.blocks = (long long)num_sms() * 8;
+        if (p.blocks > nlines) p.blocks = nlines;
+        p.per_block = ceil_div<long long>(nlines, p.blocks);
+        p.smem = ((size_t)g.ow * g.cout + (size_t)g.kd * g.kh * (g.ow + g.kw - 1) * g.cin) * sizeof(float);
     }
-    long long blocks = (long long)num_sms() * 8;
-    if (blocks > nlines) blocks = nlines;
-    const size_t smem = ((size_t)g.ow * g.cout + (size_t)g.kd * g.kh * (g.ow + g.kw - 1) * g.cin) * sizeof(float);
-    static bool attr[kMaxDevices] = {};
-    if (!ensure_smem_attr(stem_wgrad_kernel, 96 * 1024, attr)) return MDT_EDRIVER;
-    stem_wgrad_kernel<<<(unsigned)blocks, 256, smem, st>>>(g, x, dy, dw, ceil_div<long long>(nlines, blocks));
+    return p;
+}
+
+size_t conv_stem_wgrad_workspace_bytes(const ConvGeom &g) {
+    const StemWgradPlan p = stem_wgrad_plan(g);
+    const size_t w = sizeof(float) * (size_t)p.blocks * g.cout * g.cin * g.kd * g.kh * g.kw, b = conv_bias_grad_workspace_bytes(g);
+    return w > b ? w : b;
+}
+
+int conv_stem_wgrad(const ConvGeom &g, const float *x, const float *dy, float *dw, float *db, void *ws, size_t ws_bytes, cudaStream_t st) {
+    if (!ws || ws_bytes < conv_stem_wgrad_workspace_bytes(g)) return MDT_EWORKSPACE;
+    const StemWgradPlan p = stem_wgrad_plan(g);
+    float *partial = reinterpret_cast<float *>(ws);
+    if (p.c1k3) {
+        static bool attr3[kMaxDevices] = {};
+        if (!ensure_smem_attr(stem_wgrad_c1k3_kernel, 96 * 1024, attr3)) return MDT_EDRIVER;
+        stem_wgrad_c1k3_kernel<<<(unsigned)p.blocks, 256, p.smem, st>>>(g, x, dy, partial, p.per_block);
+    } else {
+        static bool attr[kMaxDevices] = {};
+        if (!ensure_smem_attr(stem_wgrad_kernel, 96 * 1024, attr)) return MDT_EDRIVER;
+        stem_wgrad_kernel<<<(unsigned)p.blocks, 256, p.smem, st>>>(g, x, dy, partial, p.per_block);
+    }
     int rc = launch_status();
     if (rc) return rc;
-    if (db) return conv_bias_grad(g, dy, db, st);
+    if ((rc = reduce_partials(partial, (int)p.blocks, (long long)g.cout * g.cin * g.kd * g.kh * g.kw, dw, st))) return rc;
+    if (db) return conv_bias_grad(g, dy, db, ws, ws_bytes, st);   // reuses the workspace after the reduction (same stream)
     return MDT_OK;
 }
 

@@ -38,20 +38,14 @@ __global__ void __launch_bounds__(256) split_rows_kernel(const float *__restrict
     // backward-pass extras, all fused into this one streaming pass over dy:
     //   relu_of    : forward output y of a conv with fused ReLU -> the element is zeroed where y <= 0 (threshold_backward)
     //   masked_out : fp32 copy of the masked gradient (needed when it is also the gradient of a fused residual input)
-    //   colsum     : [C] bias gradient, accumulated per block in shared memory, one global atomic per channel and block
-    __shared__ float s_sum[256];
+    //   colsum     : [gridDim.x][C] per-block column sums (bias-gradient partials, combined by reduce_partials); needs gridDim * 256 to be a
+    //                multiple of Cp / 8, so that a thread keeps the same 8 channels for all its rows and sums them in registers
+    __shared__ float s_part[256][8];
     const int groups = Cp / 8;  // 8 channels (16 bytes of bf16) per thread
     const long long total = rows * groups;
     const long long plane_stride = inter_w > 0 ? (long long)inter_w * Cp : rows * Cp;
-    // when the grid stride is a multiple of `groups`, a thread keeps the same 8 channels for all its rows: column sums then live in
-    // registers and touch shared memory once per thread instead of once per element
-    const bool reg_sum = colsum && ((long long)gridDim.x * blockDim.x) % groups == 0;
     const bool vec4 = (C & 3) == 0 && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(relu_of) | reinterpret_cast<uintptr_t>(masked_out)) & 15) == 0;
     float rs[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    if (colsum) {
-        for (int i = threadIdx.x; i < Cp && i < 256; i += blockDim.x) s_sum[i] = 0.f;
-        __syncthreads();
-    }
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long r = i / groups;
         const int c0 = (int)(i % groups) * 8;
@@ -87,13 +81,9 @@ __global__ void __launch_bounds__(256) split_rows_kernel(const float *__restrict
                     if (c0 + k < C) masked_out[r * C + c0 + k] = v[k];
             }
         }
-        if (reg_sum) {
+        if (colsum) {
 #pragma unroll
             for (int k = 0; k < 8; ++k) rs[k] += v[k];
-        } else if (colsum) {
-#pragma unroll
-            for (int k = 0; k < 8; ++k)
-                if (c0 + k < C && v[k] != 0.f) atomicAdd(&s_sum[c0 + k], v[k]);
         }
         __align__(16) __nv_bfloat16 hi[8], lo[8];
 #pragma unroll
@@ -107,16 +97,17 @@ __global__ void __launch_bounds__(256) split_rows_kernel(const float *__restrict
         *reinterpret_cast<uint4 *>(dst + off) = *reinterpret_cast<const uint4 *>(hi);
         if (planes > 1) *reinterpret_cast<uint4 *>(dst + off + plane_stride) = *reinterpret_cast<const uint4 *>(lo);
     }
-    if (reg_sum) {
-        const int c0 = (int)((blockIdx.x * (long long)blockDim.x + threadIdx.x) % groups) * 8;
-#pragma unroll
-        for (int k = 0; k < 8; ++k)
-            if (c0 + k < C && rs[k] != 0.f) atomicAdd(&s_sum[c0 + k], rs[k]);
-    }
     if (colsum) {
+        // thread t holds the sums of group (blockIdx.x * blockDim.x + t) % groups; channel c adds its threads up in increasing t
+#pragma unroll
+        for (int k = 0; k < 8; ++k) s_part[threadIdx.x][k] = rs[k];
         __syncthreads();
-        for (int i = threadIdx.x; i < C && i < 256; i += blockDim.x)
-            if (s_sum[i] != 0.f) atomicAdd(colsum + i, s_sum[i]);
+        const int base = (int)((blockIdx.x * (long long)blockDim.x) % groups);
+        for (int c = threadIdx.x; c < C; c += blockDim.x) {
+            float t = 0.f;
+            for (int u = ((c / 8 - base) % groups + groups) % groups; u < (int)blockDim.x; u += groups) t += s_part[u][c % 8];
+            colsum[(long long)blockIdx.x * C + c] = t;
+        }
     }
 }
 

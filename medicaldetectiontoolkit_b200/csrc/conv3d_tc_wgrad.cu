@@ -335,7 +335,9 @@ size_t conv_tc_wgrad_workspace_bytes(const ConvGeom &g, int precision) {
     const int planes = precision == 1 ? 1 : 2;
     const size_t rows_y = (size_t)g.n * g.od * g.oh * g.ow, rows_x = (size_t)g.n * g.d * g.h * g.w;
     const size_t partial = (size_t)wg_splits(g, w) * w.groups * w.mtiles * 128 * wg_slot_cols(g, w) * sizeof(float);
-    return wg_align(planes * rows_y * conv_tc_kpad(g.cout) * 2) + wg_align(planes * rows_x * conv_tc_kpad(g.cin) * 2) + wg_align(partial) + 2048;
+    const size_t b = wg_align(planes * rows_y * conv_tc_kpad(g.cout) * 2) + wg_align(planes * rows_x * conv_tc_kpad(g.cin) * 2) + wg_align(partial) + 2048;
+    const size_t bias = conv_bias_grad_workspace_bytes(g);
+    return b > bias ? b : bias;
 }
 
 // dy_presplit != nullptr: dy is already split (interleaved layout, conv_tc_kpad(cout) channels); then db must have been produced by the caller
@@ -436,7 +438,7 @@ static int conv_tc_wgrad_impl(const ConvGeom &g, const float *x, const float *dy
         wgrad_reduce_kernel<<<(unsigned)ceil_div<long long>(total, 256), 256, 0, st>>>(p, dw);
         if ((rc = launch_status())) return rc;
     }
-    if (db && !dy_presplit) return conv_bias_grad(g, dy, db, st);
+    if (db && !dy_presplit) return conv_bias_grad(g, dy, db, ws, ws_bytes, st);   // the workspace is free again once the reduction has run
     return MDT_OK;
 }
 
@@ -452,12 +454,30 @@ bool conv_tc_backward_supported(const ConvGeom &g, bool need_dx) {
     return conv_tc_wgrad_supported(g) && (!need_dx || conv_tc_supported(g, 1)) && g.cout <= 256;
 }
 
+// grid of the split pass over dy; with a bias gradient a thread must stay on the same 8-channel group across its grid-stride steps (its column
+// sums live in registers), i.e. gridDim * 256 must be a multiple of co_p / 8 (6 groups for 36 -> 48 channels)
+static long long backward_split_blocks(const ConvGeom &g, bool with_bias) {
+    const int co_p = conv_tc_kpad(g.cout);
+    const long long rows_y = (long long)g.n * g.od * g.oh * g.ow;
+    long long blocks = ceil_div<long long>(rows_y * (co_p / 8), 256);
+    if (blocks > (long long)num_sms() * 16) blocks = (long long)num_sms() * 16;
+    if (with_bias) {
+        const long long groups = co_p / 8;
+        long long unit = groups;
+        for (long long a = groups, b = 256; b;) { const long long t = a % b; a = b; b = t; unit = groups / a; }   // groups / gcd(groups, 256)
+        blocks = blocks > unit ? blocks / unit * unit : unit;
+    }
+    return blocks;
+}
+
 size_t conv_tc_backward_workspace_bytes(const ConvGeom &g, bool need_dx, int precision) {
     const int planes = precision == 1 ? 1 : 2;
     const size_t rows_y = (size_t)g.n * g.od * g.oh * g.ow;
     const size_t ys = wg_align(planes * rows_y * conv_tc_kpad(g.cout) * 2);
     size_t inner = conv_tc_wgrad_workspace_bytes(g, precision);
     if (need_dx) { const size_t d = conv_tc_workspace_bytes(g, 1, precision); if (d > inner) inner = d; }
+    const size_t colsum = sizeof(float) * (size_t)backward_split_blocks(g, true) * g.cout;   // per-block bias-gradient partials
+    if (colsum > inner) inner = colsum;
     return ys + inner + 4096;
 }
 
@@ -472,23 +492,14 @@ int conv_tc_backward(const ConvGeom &g, const float *x, const float *dy, const f
     __nv_bfloat16 *ys = reinterpret_cast<__nv_bfloat16 *>(base);
     uint8_t *inner = base + wg_align((size_t)planes * rows_y * co_p * 2);
     const size_t inner_bytes = ws_bytes - (size_t)(inner - reinterpret_cast<uint8_t *>(ws));
-    if (db) {
-        cudaError_t e = cudaMemsetAsync(db, 0, sizeof(float) * g.cout, st);
-        if (e != cudaSuccess) return (int)e;
-    }
-    long long blocks = ceil_div<long long>(rows_y * (co_p / 8), 256);
-    if (blocks > (long long)num_sms() * 16) blocks = (long long)num_sms() * 16;
-    if (db) {
-        // the kernel keeps the column sums (bias gradient) in registers only if a thread stays on the same 8-channel group across its grid-stride
-        // steps, i.e. gridDim * 256 is a multiple of co_p / 8 (6 groups for 36 -> 48 channels): round the grid down to such a size
-        const long long groups = co_p / 8;
-        long long unit = groups;
-        for (long long a = groups, b = 256; b;) { const long long t = a % b; a = b; b = t; unit = groups / a; }   // groups / gcd(groups, 256)
-        if (blocks > unit) blocks = blocks / unit * unit;
-    }
-    split_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(dy, ys, rows_y, g.cout, co_p, planes, g.ow, relu_of, dy_masked_out, db);
+    const long long blocks = backward_split_blocks(g, db != nullptr);
+    // bias gradient: per-block column sums go to the (not yet used) inner workspace and are combined in a fixed order before dgrad / wgrad
+    // reuse that memory
+    float *colsum = db ? reinterpret_cast<float *>(inner) : nullptr;
+    split_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(dy, ys, rows_y, g.cout, co_p, planes, g.ow, relu_of, dy_masked_out, colsum);
     int rc = launch_status();
     if (rc) return rc;
+    if (db && (rc = reduce_partials(colsum, (int)blocks, g.cout, db, st))) return rc;
     if (dx && (rc = conv_tc_run(g, 1, nullptr, w, nullptr, nullptr, dx, 0, precision, inner, inner_bytes, st, ys, nullptr))) return rc;
     return conv_tc_wgrad_impl(g, x, nullptr, dw, nullptr, precision, inner, inner_bytes, st, ys, reinterpret_cast<const __nv_bfloat16 *>(x_split));
 }

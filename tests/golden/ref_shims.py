@@ -174,3 +174,32 @@ def ref_cf(cf):
     c.backbone_path = os.path.join(REF, "models", "backbone.py")
     c.scale = np.asarray(c.scale)
     return c
+
+
+def drop_cuda_functions():
+    """forget the injected / drop-in `cuda_functions` modules"""
+    for k in [k for k in sys.modules if k == "cuda_functions" or k.startswith("cuda_functions.")]:
+        del sys.modules[k]
+
+
+def dropin_setup(model, patch=(64, 64, 32)):
+    """the reference's graph on this package (INTEGRATION.md §1): `install_dropin()` + the two `mutils` attribute patches + `cf.backbone_path`
+    pointing at this package's backbone.py.  Returns (mutils, saved, cf); undo with dropin_teardown(mutils, saved)."""
+    import medicaldetectiontoolkit_b200 as mdt
+    from medicaldetectiontoolkit_b200 import conv as b200_conv
+    from medicaldetectiontoolkit_b200 import model_utils as b200_mutils
+    from medicaldetectiontoolkit_b200.configs import make_cf
+    install_import_shims()          # matplotlib stubs + sys.path (its oracle-backed cuda_functions are replaced on the next line)
+    mdt.install_dropin()
+    import utils.model_utils as mutils
+    saved = (mutils.NDConvGenerator, mutils.gt_anchor_matching)
+    mutils.NDConvGenerator = b200_conv.NDConvGenerator
+    mutils.gt_anchor_matching = b200_mutils.gt_anchor_matching
+    cf = ref_cf(make_cf(model, 3, patch))
+    cf.backbone_path = os.path.join(ROOT, "medicaldetectiontoolkit_b200", "backbone.py")
+    return mutils, saved, cf
+
+
+def dropin_teardown(mutils, saved):
+    mutils.NDConvGenerator, mutils.gt_anchor_matching = saved
+    drop_cuda_functions()

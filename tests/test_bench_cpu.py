@@ -24,3 +24,30 @@ def test_roofline_object_has_the_contract_keys():
     r2 = bench.make_roofline(3.6e12, 52.0, 229, 66.7, None, 1400.0, False)
     assert r2["traffic"] is None and "fallback" in r2["peak_source"] and r2["frac"] == r2["all_conv_launches"]["frac"]
     assert bench.make_roofline(3.6e12, None, 0, 66.7, None, 1400.0, False) is None
+
+
+def test_step_outputs_are_float_copies_and_large_arrays_are_sampled(monkeypatch):
+    import numpy as np
+    import torch
+    net = torch.nn.Sequential(torch.nn.Linear(4, 3), torch.nn.Linear(3, 2))
+    seg = np.zeros((2, 1, 4, 4, 2), dtype=np.uint8)
+    seg[1, 0, 2] = 1
+    res = {'torch_loss': torch.tensor([1.5]), 'monitor_values': {'loss': 1.5, 'class_loss': 0.25}, 'seg_preds': seg,
+           'boxes': [[{'box_coords': np.array([1, 2, 3, 4, 0, 1]), 'box_label': 1, 'box_type': 'gt'}],
+                     [{'box_coords': np.array([5, 6, 9, 9, 1, 2], dtype=np.int32), 'box_score': np.float32(0.75), 'box_type': 'det',
+                       'box_pred_class_id': np.int32(1)}]]}
+    out = bench.step_outputs(res, net, 3)
+    assert sorted(out) == ["detections", "loss", "monitor_class_loss", "monitor_loss", "parameters", "seg_preds"]
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    assert out["detections"].tolist() == [[1, 5, 6, 9, 9, 1, 2, 1, 0.75]]
+    assert out["loss"].tolist() == [1.5] and out["monitor_class_loss"].tolist() == [0.25]
+    seg[:] = 7                                                    # the step's host buffer is reused by the next step
+    assert out["seg_preds"].shape == (2, 1, 4, 4, 2) and out["seg_preds"].sum() == 8
+    flat = torch.cat([p.detach().reshape(-1) for p in net.parameters()]).numpy()
+    assert np.array_equal(out["parameters"], flat)
+    monkeypatch.setattr(bench, "DUMP_MAX_ELEMS", 10)
+    a, b = bench.step_outputs(res, net, 3), bench.step_outputs(res, net, 3)
+    assert a["parameters"].shape == (10,) and np.array_equal(a["parameters"], b["parameters"])   # fixed sample
+    assert np.all(np.isin(a["parameters"], flat)) and a["seg_preds"].shape == (10,)
+    empty = dict(res, boxes=[[], []])
+    assert bench.step_outputs(empty, net, 3)["detections"].shape == (0, 9)

@@ -274,3 +274,29 @@ def test_full_resolution_layers_vs_fp64(cin, cout, k, stride, pad):
     ref.backward(gy.double().contiguous())
     errs = {"fprop": _rel(y, ref.detach()), "dgrad": _rel(dx, xd.grad), "wgrad": _rel(dw, wd.grad), "bias": _rel(db, bd.grad)}
     assert errs["fprop"] < 3e-5 and errs["dgrad"] < 3e-5 and errs["wgrad"] < 3e-5 and errs["bias"] < 3e-5, errs
+
+
+@pytest.mark.parametrize("cin,cout,k,sp,algo", [(1, 18, 3, (8, 8, 128), 0),     # stem, c1k3 weight-gradient kernel
+                                                (2, 18, 3, (4, 4, 16), 0),      # stem, generic kernel
+                                                (18, 18, 3, (8, 8, 32), 1),     # fp32 SIMT split-M weight gradient
+                                                (36, 36, 3, (8, 16, 128), 2),   # tcgen05 weight gradient + bias_grad_kernel
+                                                (288, 576, 1, (4, 4, 8), 0)])   # wide bias gradient (cout > 256)
+def test_weight_and_bias_gradients_are_bitwise_reproducible(cin, cout, k, sp, algo):
+    """the cross-block reductions of the weight / bias gradients combine per-block partials in a fixed order (no float atomics): the same
+    inputs give the same bits on every call, through both the unfused wgrad and the fused backward"""
+    g = torch.Generator(device=DEV).manual_seed(cin * 1000 + cout)
+    x = torch.randn((2, cin) + sp, device=DEV, generator=g).contiguous(memory_format=torch.channels_last_3d)
+    w = torch.randn(cout, cin, k, k, k, device=DEV, generator=g) * 0.05
+    gy = torch.randn((2, cout) + sp, device=DEV, generator=g).contiguous(memory_format=torch.channels_last_3d)
+    p3 = (k // 2,) * 3
+    first = C.conv3d_wgrad(x, gy, tuple(w.shape), (1, 1, 1), p3, True, algo=algo)
+    for _ in range(3):
+        again = C.conv3d_wgrad(x, gy, tuple(w.shape), (1, 1, 1), p3, True, algo=algo)
+        assert torch.equal(first[0], again[0]) and torch.equal(first[1], again[1])
+    fused = C.conv3d_backward(x, gy, None, w, (1, 1, 1), p3, True, True, False, algo=algo)
+    if fused is not None:
+        for _ in range(3):
+            again = C.conv3d_backward(x, gy, None, w, (1, 1, 1), p3, True, True, False, algo=algo)
+            assert all(torch.equal(a, b) for a, b in zip(fused[:3], again[:3]))
+        ref_db = gy.double().sum(dim=(0, 2, 3, 4))
+        assert float((fused[2].double() - ref_db).abs().max() / ref_db.abs().max()) < TOL

@@ -240,3 +240,32 @@ def test_retina_forward_matches_cpu_port(dim, patch):
     order_g = np.lexsort((got[:, -1].numpy(), got[:, 2 * dim].numpy()))
     order_r = np.lexsort((det_r[:, -1].numpy(), det_r[:, 2 * dim].numpy()))
     assert np.allclose(got.numpy()[order_g], det_r.numpy()[order_r], atol=1e-5)
+
+
+def test_train_steps_are_bitwise_reproducible():
+    """two independent runs of two Retina U-Net train steps (forward, matching, losses, detections, backward, Adam) from the same seeds
+    compute the same bits: losses, detections, segmentation and the updated parameters"""
+    from medicaldetectiontoolkit_b200 import retina_unet
+    cf = make_cf('retina_unet', 3, (64, 64, 32))
+
+    def run():
+        torch.manual_seed(0)
+        np.random.seed(0)
+        net = retina_unet.net(cf, None).to(DEV)
+        opt = torch.optim.Adam(net.parameters(), lr=1e-4)
+        out = []
+        for i in range(2):
+            res = net.train_forward(synthetic_batch(cf, 2, seed=i))
+            opt.zero_grad()
+            res['torch_loss'].backward()
+            opt.step()
+            dets = [[b] + [float(c) for c in bx['box_coords']] + [float(bx['box_score'])]
+                    for b, boxes in enumerate(res['boxes']) for bx in boxes if bx['box_type'] == 'det']
+            out.append((float(res['torch_loss']), dets, np.array(res['seg_preds'], copy=True)))
+        params = torch.cat([p.detach().reshape(-1) for p in net.parameters()]).cpu()
+        return out, params
+
+    (a, pa), (b, pb) = run(), run()
+    for (la, da, sa), (lb, db, sb) in zip(a, b):
+        assert la == lb and da == db and np.array_equal(sa, sb)
+    assert torch.equal(pa, pb)

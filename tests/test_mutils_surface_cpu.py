@@ -1,6 +1,7 @@
 """The small host-side helpers that complete the `mutils` surface (model_utils.py: compute_iou_*, compute_overlaps, clip_boxes_numpy,
-intersect1d, sum_tensor, get_dice_per_batch_and_class, batch_dice_mask, unmold_mask_*) against the reference's own functions, imported
-unmodified from /root/reference (build container only; skipped where the tree is absent)."""
+intersect1d, sum_tensor, get_dice_per_batch_and_class, batch_dice_mask, unmold_mask_*) against the reference's own functions: their outputs
+on the seeded inputs of make_mutils_golden.py are stored in tests/golden/mutils_surface.npz (bit-identical ones as digests)."""
+import json
 import os
 import sys
 
@@ -10,63 +11,40 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
-REF = os.environ.get("REF", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "utils")), reason="reference tree not present")
+import make_mutils_golden as MG  # noqa: E402
+from digest import digest  # noqa: E402
 
 from medicaldetectiontoolkit_b200 import model_utils as M  # noqa: E402
 
 
 @pytest.fixture(scope="module")
-def ref():
-    import ref_shims as RS
-    RS.install_import_shims()
-    import utils.model_utils as mutils
-    return mutils
-
-
-def _boxes(rs, n, dim):
-    lo = rs.uniform(0, 100, size=(n, dim))
-    hi = lo + rs.uniform(1, 40, size=(n, dim))
-    return np.concatenate([lo[:, :2], hi[:, :2]] + ([lo[:, 2:], hi[:, 2:]] if dim == 3 else []), axis=1)[:, [0, 1, 2, 3] + ([4, 5] if dim == 3 else [])]
+def ref(golden_dir):
+    g = np.load(os.path.join(golden_dir, "mutils_surface.npz"))
+    return {k: json.loads(str(g[k])) if g[k].dtype.kind == "U" else g[k] for k in g.files}
 
 
 @pytest.mark.parametrize("dim", [2, 3])
 def test_numpy_iou_helpers_bit_identical(ref, dim):
-    rs = np.random.RandomState(dim)
-    a, b = _boxes(rs, 300, dim), _boxes(rs, 17, dim)
-    assert np.array_equal(M.compute_overlaps(a, b), ref.compute_overlaps(a, b))
-    vol = np.prod(a[:, [2, 3] + ([5] if dim == 3 else [])] - a[:, [0, 1] + ([4] if dim == 3 else [])], axis=1)
-    vb = float(np.prod(b[0, [2, 3] + ([5] if dim == 3 else [])] - b[0, [0, 1] + ([4] if dim == 3 else [])]))
-    f, g = (M.compute_iou_2D, ref.compute_iou_2D) if dim == 2 else (M.compute_iou_3D, ref.compute_iou_3D)
-    assert np.array_equal(f(b[0], a, vb, vol), g(b[0], a, vb, vol))
-    win = (64, 80) if dim == 2 else (64, 80, 48)
-    wild = a * 1.7 - 30
-    assert np.array_equal(M.clip_boxes_numpy(wild, win), ref.clip_boxes_numpy(wild, win))
+    i = MG.iou_inputs(dim)
+    a, b = i["a"], i["b"]
+    assert digest(M.compute_overlaps(a, b)) == ref["iou%d__overlaps" % dim]
+    f = M.compute_iou_2D if dim == 2 else M.compute_iou_3D
+    assert digest(f(b[0], a, float(i["vb"][0]), i["vol"])) == ref["iou%d__iou" % dim]
+    assert digest(M.clip_boxes_numpy(i["wild"], tuple(i["win"].tolist()))) == ref["iou%d__clip" % dim]
 
 
 def test_tensor_helpers(ref):
-    rs = np.random.RandomState(5)
-    t1, t2 = torch.from_numpy(rs.permutation(50)[:20]), torch.from_numpy(rs.permutation(50)[:25])
-    assert torch.equal(M.intersect1d(t1, t2), ref.intersect1d(t1, t2))
-    x = torch.from_numpy(rs.rand(2, 3, 4, 5, 6))
-    for axes in [(0, 2, 3, 4), (1,), (0, 2)]:
-        assert torch.allclose(M.sum_tensor(x, axes), ref.sum_tensor(x, axes), rtol=1e-13, atol=0)
-        assert M.sum_tensor(x, axes, keepdim=True).shape == ref.sum_tensor(x, axes, keepdim=True).shape
-    pred, y = rs.randint(0, 3, (2, 1, 8, 8, 4)), rs.randint(0, 3, (2, 1, 8, 8, 4))
-    assert np.allclose(M.get_dice_per_batch_and_class(pred, y, 3), ref.get_dice_per_batch_and_class(pred, y, 3), rtol=1e-14)
-    p2 = torch.softmax(torch.from_numpy(rs.randn(2, 2, 8, 8)), 1)
-    y2 = torch.nn.functional.one_hot(torch.from_numpy(rs.randint(0, 2, (2, 8, 8))), 2).movedim(-1, 1).double()
-    m2 = torch.from_numpy((rs.rand(2, 8, 8) > 0.3).astype(np.float64))
-    assert abs(float(M.batch_dice_mask(p2, y2, m2)) - float(ref.batch_dice_mask(p2, y2, m2))) < 1e-14
-    p3 = torch.softmax(torch.from_numpy(rs.randn(1, 2, 4, 4, 4)), 1)
-    y3 = torch.nn.functional.one_hot(torch.from_numpy(rs.randint(0, 2, (1, 4, 4, 4))), 2).movedim(-1, 1).double()
-    assert abs(float(M.batch_dice_mask(p3, y3, None)) - float(M.batch_dice(p3, y3))) < 1e-15
+    t = {k: torch.from_numpy(v) for k, v in MG.tensor_inputs().items()}
+    assert torch.equal(M.intersect1d(t["t1"], t["t2"]), torch.from_numpy(ref["tensor__intersect1d"]))
+    for j, axes in enumerate(MG.SUM_AXES):
+        assert torch.allclose(M.sum_tensor(t["x"], axes), torch.from_numpy(ref["tensor__sum_%d" % j]), rtol=1e-13, atol=0)
+        assert list(M.sum_tensor(t["x"], axes, keepdim=True).shape) == ref["tensor__sum_keepdim_shape_%d" % j].tolist()
+    assert np.allclose(M.get_dice_per_batch_and_class(t["pred"].numpy(), t["y"].numpy(), 3), ref["tensor__dice"], rtol=1e-14)
+    assert abs(float(M.batch_dice_mask(t["p2"], t["y2"], t["m2"])) - float(ref["tensor__dice_mask"][0])) < 1e-14
+    assert abs(float(M.batch_dice_mask(t["p3"], t["y3"], None)) - float(M.batch_dice(t["p3"], t["y3"]))) < 1e-15
 
 
 def test_unmold_masks(ref):
-    rs = np.random.RandomState(6)
-    m2 = rs.rand(28, 28).astype(np.float32)
-    assert np.array_equal(M.unmold_mask_2D(m2, [3, 5, 40, 33], (64, 64)), ref.unmold_mask_2D(m2, [3, 5, 40, 33], (64, 64)))
-    m3 = rs.rand(14, 14, 5).astype(np.float32)
-    box = [2, 4, 30, 25, 1, 9]
-    assert np.array_equal(M.unmold_mask_3D(m3, box, (32, 32, 16)), ref.unmold_mask_3D(m3, box, (32, 32, 16)))
+    u = MG.unmold_inputs()
+    assert digest(M.unmold_mask_2D(u["m2"], u["box2"].tolist(), tuple(u["shape2"].tolist()))) == ref["unmold__out2"]
+    assert digest(M.unmold_mask_3D(u["m3"], u["box3"].tolist(), tuple(u["shape3"].tolist()))) == ref["unmold__out3"]

@@ -1,6 +1,6 @@
 """GPU parity tests (run on the B200 with -m gpu): every call goes through the C-ABI of libmdt_b200.so and is compared with
  (a) the CPU oracle (oracle/mdt_oracle.c, oracle/matching_oracle.py), (b) the committed golden fixtures, and
- (c) the reference's own unmodified kernels compiled for sm_100a (oracle/_ref), when that build is present.
+ (c) the reference's own unmodified kernels compiled for sm_100a (oracle/_ref), through their stored outputs (tests/golden/ref_*.npz).
 Tolerances: NMS keep indices and anchor labels bit-exact; RoIAlign 1e-4 relative to max|ref| (north_star)."""
 import os
 import sys
@@ -14,6 +14,7 @@ import _oracle as O
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import make_ref_kernel_golden as RK  # noqa: E402
 import matching_oracle as MO  # noqa: E402
 from golden_cfg import cf2d, cf3d  # noqa: E402
 
@@ -83,19 +84,20 @@ def test_nms_dropin_api_and_mask():
         NO.nms_sorted(torch.zeros(4, 7), 0.5, 3)  # CPU tensor: no fallback
 
 
-def test_nms_full_size_cfg4_properties_and_reference_kernel():
-    """BASELINE cfg4: 100 k boxes, IoU 0.5.  Size-independent properties + equality with the reference's own kernel + host scan."""
-    for n, thr, rounded in [(100000, 0.5, True), (50000, 1e-5, True), (6000, 0.7, False)]:
+def test_nms_full_size_cfg4_properties_and_reference_kernel(golden_dir):
+    """BASELINE cfg4: 100 k boxes, IoU 0.5.  Size-independent properties + equality with the reference's own kernel + host scan
+    (its keep lists on the same inputs, tests/golden/ref_nms.npz from make_ref_kernel_golden.py)."""
+    g = np.load(os.path.join(golden_dir, "ref_nms.npz"))
+    for n, thr, rounded in RK.NMS_3D_CASES:
         b = O.synth_boxes(n, 3, seed=n, rounded=rounded)
         keep = _keep(b, thr, 3)
         assert keep[0] == 0 and np.all(np.diff(keep) > 0)          # sorted, first box always kept
         again = _keep(b[keep], thr, 3)
         assert again.tolist() == list(range(len(keep)))            # idempotence: survivors do not suppress each other
-        if O.ref_lib("nms3d") is not None:
-            assert keep.tolist() == O.ref_nms(b, thr, 3).tolist()  # bit-identical to the reference kernel on the same GPU
-    if O.ref_lib("nms2d") is not None:
-        b = O.synth_boxes(30000, 2, seed=3, rounded=False)
-        assert _keep(b, 0.5, 2).tolist() == O.ref_nms(b, 0.5, 2).tolist()
+        assert keep.tolist() == RK.kept(g["nms3d_%d" % n], n).tolist()   # bit-identical to the reference kernel
+    n, thr, rounded, seed = RK.NMS_2D_CASE
+    b = O.synth_boxes(n, 2, seed=seed, rounded=rounded)
+    assert _keep(b, thr, 2).tolist() == RK.kept(g["nms2d_%d" % n], n).tolist()
 
 
 # ----------------------------------------------------------------------------------------------------------------------------------- RoIAlign
@@ -133,32 +135,40 @@ def test_roi_align_forward_backward_vs_oracle(dim, shape, crop):
         assert _rel(x.grad.cpu().numpy(), want_gx) < 1e-4, layout
 
 
-def test_roi_align_vs_reference_kernels_cfg3():
-    """cfg3 shapes: 36-channel FPN maps, 512 boxes per image x 2, pools (7,7,3) and (14,14,5); compared with the reference's own kernels"""
-    if O.ref_lib("roi3d") is None:
-        pytest.skip("oracle/_ref not built")
-    rs = np.random.RandomState(4)
-    for shape, crop in [((2, 36, 32, 32, 128), (7, 7, 3)), ((2, 36, 16, 16, 64), (14, 14, 5)), ((2, 36, 4, 4, 16), (7, 7, 3))]:
-        img = rs.randn(*shape).astype(np.float32)
-        boxes, ind = O.synth_rois(1024, 3, 2, seed=8)
-        ref = O.ref_crop_and_resize_forward(img, boxes, ind, crop)
-        fn = NO.CropAndResizeFunction(*crop, 0)
-        for cl in (False, True):
+def test_roi_align_vs_reference_kernels_cfg3(golden_dir):
+    """cfg3 shapes: 36-channel FPN maps, 512 boxes per image x 2, pools (7,7,3) and (14,14,5); compared with the reference's own kernels
+    (seeded samples of their outputs on the same inputs, tests/golden/ref_roi_align.npz from make_ref_kernel_golden.py; where oracle/_ref is
+    built, also whole arrays against the kernels themselves)"""
+    g = np.load(os.path.join(golden_dir, "ref_roi_align.npz"))
+    live = O.ref_lib("roi3d") is not None and O.ref_lib("roi2d") is not None
+    full = {}
+
+    def check(tag, got, tol):
+        assert list(got.shape) == g[tag + "__shape"].tolist(), tag
+        err = np.abs(got.reshape(-1)[RK.sample_ix(got.size, tag)].astype(np.float64) - g[tag + "__sample"]).max() / g[tag + "__maxabs"][0]
+        assert err < tol, (tag, err)
+        if live:
+            assert _rel(got, full[tag]) < tol, tag
+
+    for tag, kind, args in RK.roi_inputs():
+        if live:
+            full[tag] = RK.ref_output(kind, args)
+        if kind == "fwd3":
+            img, boxes, ind, crop = args
+            fn, fwd_tag = NO.CropAndResizeFunction(*crop, 0), tag
+        elif kind == "bwd3":
+            gy, boxes, ind, shape, layout = args
             x = torch.from_numpy(img).to(DEV)
-            x = x.contiguous(memory_format=torch.channels_last_3d) if cl else x
+            x = x.contiguous(memory_format=torch.channels_last_3d) if layout == "channels_last" else x
             x.requires_grad_(True)
             y = fn(x, torch.from_numpy(boxes).to(DEV), torch.from_numpy(ind).to(DEV))
-            assert _rel(y.detach().cpu().numpy(), ref) < 1e-5
-            gy = rs.randn(*ref.shape).astype(np.float32)
+            check(fwd_tag, y.detach().cpu().numpy(), 1e-5)
             y.backward(torch.from_numpy(gy).to(DEV))
-            ref_g = O.ref_crop_and_resize_backward(gy, boxes, ind, shape)
-            assert _rel(x.grad.cpu().numpy(), ref_g) < 1e-4  # fp32 atomics reorder on both sides
-    if O.ref_lib("roi2d") is not None:
-        img = rs.randn(2, 36, 64, 64).astype(np.float32)
-        boxes, ind = O.synth_rois(300, 2, 2, seed=9)
-        ref = O.ref_crop_and_resize_forward(img, boxes, ind, (7, 7))
-        y = NO.CropAndResizeFunction2D(7, 7, 0)(torch.from_numpy(img).to(DEV), torch.from_numpy(boxes).to(DEV), torch.from_numpy(ind).to(DEV))
-        assert _rel(y.cpu().numpy(), ref) < 1e-5
+            check(tag, x.grad.cpu().numpy(), 1e-4)  # fp32 atomics reorder on both sides
+        else:
+            img2, boxes, ind, crop = args
+            y = NO.CropAndResizeFunction2D(*crop, 0)(torch.from_numpy(img2).to(DEV), torch.from_numpy(boxes).to(DEV), torch.from_numpy(ind).to(DEV))
+            check(tag, y.cpu().numpy(), 1e-5)
 
 
 def test_roi_align_gt_mask_call_shape():

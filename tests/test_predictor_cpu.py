@@ -1,13 +1,13 @@
 """Patient-level prediction pipeline (medicaldetectiontoolkit_b200/predictor.py: Predictor) against the reference's unmodified `Predictor`
-(predictor.py:27-510) driven by the SAME deterministic stand-in network on the CPU: chunked forwarding, re-tiling of boxes and segmentation
-into patient coordinates (float16 sums, overlap counts), patch ids / centre factors / overlap counts per box, the three test-time mirrorings,
-and the consolidation calls.  The consolidation kernels need a GPU, so here `weighted_box_clustering` / `nms_2to3D` are bound to the CPU
-restatement of the kernels' formulation (oracle/consolidate_oracle.py, itself pinned to reference goldens in test_consolidate_cpu.py).
-Needs the reference tree (build container); skipped where it is absent."""
+(predictor.py:27-510) driven by the SAME deterministic stand-in network on the CPU (tests/golden/predictor_standin.py; the reference's
+outputs are stored in tests/golden/predictor.npz by make_predictor_golden.py, segmentations as digests): chunked forwarding, re-tiling of
+boxes and segmentation into patient coordinates (float16 sums, overlap counts), patch ids / centre factors / overlap counts per box, the
+three test-time mirrorings, and the consolidation calls.  The consolidation kernels need a GPU, so here `weighted_box_clustering` /
+`nms_2to3D` are bound to the CPU restatement of the kernels' formulation (oracle/consolidate_oracle.py, itself pinned to reference goldens in test_consolidate_cpu.py)."""
 import copy
+import json
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
@@ -15,81 +15,20 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
-REF = os.environ.get("REF", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "predictor.py")), reason="reference tree not present")
 
 from medicaldetectiontoolkit_b200 import predictor as P  # noqa: E402
-
-
-class Logger:
-    def info(self, *a, **k):
-        pass
-
-
-class StandInNet:
-    """deterministic function of the input patch: a few boxes per batch element + a label map; fresh dicts on every call"""
-
-    def __init__(self, dim):
-        self.dim = dim
-
-    def parameters(self):
-        return iter(())
-
-    def _element(self, patch):
-        rs = np.random.RandomState(int(np.abs(patch).sum() * 1000) % (2 ** 31))
-        sp = patch.shape[1:]
-        boxes = []
-        for _ in range(rs.randint(1, 5)):
-            lo = [rs.randint(0, s - 6) for s in sp]
-            hi = [l + rs.randint(3, min(s - l, 12)) for l, s in zip(lo, sp)]
-            coords = [lo[0], lo[1], hi[0], hi[1]] + ([lo[2], hi[2]] if self.dim == 3 else [])
-            boxes.append({'box_coords': np.array(coords, dtype=np.int32), 'box_score': float(rs.uniform(0.1, 0.99)), 'box_type': 'det',
-                          'box_pred_class_id': int(rs.randint(1, 3))})
-        return boxes
-
-    def test_forward(self, batch, return_masks=True):
-        data = batch['data']
-        return {'boxes': [self._element(p) for p in data], 'seg_preds': (data[:, :1] > 0.6).astype(np.uint8)}
-
-    def train_forward(self, batch, is_validation=False):
-        out = self.test_forward(batch)
-        for b in out['boxes']:
-            b.append({'box_coords': np.zeros(2 * self.dim), 'box_label': 1, 'box_type': 'gt'})
-        out['monitor_values'] = {'loss': float(batch['data'].mean()), 'class_loss': float(batch['data'].std())}
-        return out
-
-
-def _cf(dim, tmp, test_aug=False):
-    return types.SimpleNamespace(dim=dim, batch_size=3, patch_size=[32, 32, 16][:dim], test_aug=test_aug, class_dict={1: 'a', 2: 'b'}, wcs_iou=1e-5,
-                                 merge_2D_to_3D_preds=dim == 2, merge_3D_iou=0.1, return_masks_in_test=False, fold_dir=str(tmp), fold=0, test_n_epochs=2,
-                                 hold_out_test_set=False, folds=[0], exp_dir=str(tmp))
-
-
-def _patient_3d(rs):
-    shape = (1, 1, 48, 48, 24)
-    crops = [[y, y + 32, x, x + 32, z, z + 16] for y in (0, 16) for x in (0, 16) for z in (0, 8)]
-    vol = rs.rand(*shape).astype(np.float32)
-    data = np.stack([vol[0, :, c[0]:c[1], c[2]:c[3], c[4]:c[5]] for c in crops])
-    return {'data': data, 'patch_crop_coords': crops, 'original_img_shape': shape, 'pid': 'p3',
-            'patient_bb_target': np.array([[[5, 5, 20, 20, 2, 9]]]), 'patient_roi_labels': np.array([[1]])}
-
-
-def _patient_2d(rs):
-    n_slices = 5
-    shape = (n_slices, 1, 48, 48)
-    crops = [[y, y + 32, x, x + 32, z, z + 1] for z in range(n_slices) for y in (0, 16) for x in (0, 16)]
-    vol = rs.rand(*shape).astype(np.float32)
-    data = np.stack([vol[c[4], :, c[0]:c[1], c[2]:c[3]] for c in crops])
-    return {'data': data, 'patch_crop_coords': crops, 'original_img_shape': shape, 'pid': 'p2',
-            'patient_bb_target': np.array([[[5, 5, 20, 20]]] * n_slices), 'patient_roi_labels': np.array([[1]] * n_slices)}
+from digest import digest  # noqa: E402
+from predictor_standin import Logger, StandInNet, make_cf, patient, plain, whole_image  # noqa: E402
 
 
 @pytest.fixture(scope="module")
-def ref_predictor():
-    import ref_shims as RS
-    RS.install_import_shims()
-    import predictor as ref
-    return ref
+def ref_golden(golden_dir):
+    g = np.load(os.path.join(golden_dir, "predictor.npz"))
+
+    def case(name):
+        """the reference Predictor's result of one case; 'seg_preds' is the digest [shape, dtype, sha256] of its segmentation"""
+        return json.loads(str(g[name]))
+    return case
 
 
 @pytest.fixture()
@@ -113,46 +52,40 @@ def _same_boxes(ours, theirs, rtol=1e-12):
 
 
 @pytest.mark.parametrize("dim", [3, 2])
-def test_spatial_tiling_equals_the_reference(ref_predictor, tmp_path, dim):
-    rs = np.random.RandomState(dim)
-    batch = _patient_3d(rs) if dim == 3 else _patient_2d(rs)
-    cf = _cf(dim, tmp_path)
-    ours, theirs = P.Predictor(cf, StandInNet(dim), Logger(), 'val'), ref_predictor.Predictor(cf, StandInNet(dim), Logger(), 'val')
-    ours.patched_patient = theirs.patched_patient = True
+def test_spatial_tiling_equals_the_reference(ref_golden, tmp_path, dim):
+    batch = patient(dim, seed=dim)
+    b = ref_golden("tiling%d" % dim)
+    ours = P.Predictor(make_cf(dim, tmp_path), StandInNet(dim), Logger(), 'val')
+    ours.patched_patient = True
     a = ours.spatial_tiling_forward(copy.deepcopy(batch), batch['patch_crop_coords'])
-    b = theirs.spatial_tiling_forward(copy.deepcopy(batch), batch['patch_crop_coords'])
     _same_boxes(a['boxes'], b['boxes'])
-    assert a['seg_preds'].dtype == b['seg_preds'].dtype == np.float16 and np.array_equal(a['seg_preds'], b['seg_preds'])
+    assert a['seg_preds'].dtype == np.float16 and digest(a['seg_preds']) == b['seg_preds']
     assert a['monitor_values'] == b['monitor_values']
     # whole-image prediction (no patch crops): the image is one patch with overlap 1
-    whole = {'data': batch['data'][:2], 'original_img_shape': (2,) + batch['data'].shape[1:], 'pid': 'w'}
-    _same_boxes(ours.spatial_tiling_forward(copy.deepcopy(whole))['boxes'], theirs.spatial_tiling_forward(copy.deepcopy(whole))['boxes'])
+    _same_boxes(ours.spatial_tiling_forward(copy.deepcopy(whole_image(batch)))['boxes'], b['whole_boxes'])
 
 
 @pytest.mark.parametrize("dim", [3, 2])
-def test_predict_patient_val_mode_equals_the_reference(ref_predictor, tmp_path, cpu_consolidation, dim):
-    rs = np.random.RandomState(10 + dim)
-    batch = _patient_3d(rs) if dim == 3 else _patient_2d(rs)
-    cf = _cf(dim, tmp_path)
-    a = P.Predictor(cf, StandInNet(dim), Logger(), 'val').predict_patient(copy.deepcopy(batch))
-    b = ref_predictor.Predictor(cf, StandInNet(dim), Logger(), 'val').predict_patient(copy.deepcopy(batch))
+def test_predict_patient_val_mode_equals_the_reference(ref_golden, tmp_path, cpu_consolidation, dim):
+    batch = patient(dim, seed=10 + dim)
+    a = P.Predictor(make_cf(dim, tmp_path), StandInNet(dim), Logger(), 'val').predict_patient(copy.deepcopy(batch))
+    b = ref_golden("val%d" % dim)
     _same_boxes(a['boxes'], b['boxes'], rtol=1e-9)            # after weighted box clustering (and the 2D -> 3D merge for dim 2)
-    assert np.array_equal(a['seg_preds'], b['seg_preds']) and a['monitor_values'] == b['monitor_values']
+    assert digest(a['seg_preds']) == b['seg_preds'] and a['monitor_values'] == b['monitor_values']
 
 
-def test_test_mode_mirroring_and_test_set_loop(ref_predictor, tmp_path, cpu_consolidation):
+def test_test_mode_mirroring_and_test_set_loop(ref_golden, tmp_path, cpu_consolidation):
     import torch
-    rs = np.random.RandomState(7)
-    cf = _cf(3, tmp_path, test_aug=True)
+    cf = make_cf(3, tmp_path, test_aug=True)
     np.save(os.path.join(str(tmp_path), 'epoch_ranking.npy'), np.array([4, 9, 2]))
-    batch = _patient_3d(rs)
-    ours, theirs = P.Predictor(cf, StandInNet(3), Logger(), 'test'), ref_predictor.Predictor(cf, StandInNet(3), Logger(), 'test')
-    assert ours.n_ens == theirs.n_ens == 8 and list(ours.epoch_ranking) == list(theirs.epoch_ranking)
-    a, b = ours.predict_patient(copy.deepcopy(batch)), theirs.predict_patient(copy.deepcopy(batch))
+    batch = patient(3, seed=7)
+    ours, b = P.Predictor(cf, StandInNet(3), Logger(), 'test'), ref_golden("test3")
+    assert ours.n_ens == b['n_ens'] == 8 and plain(list(ours.epoch_ranking)) == b['epoch_ranking']
+    a = ours.predict_patient(copy.deepcopy(batch))
     _same_boxes(a['boxes'], b['boxes'])
-    assert a['seg_preds'].shape == b['seg_preds'].shape == (1, 4, 48, 48, 24) and np.array_equal(a['seg_preds'], b['seg_preds'])
-    assert ours.__class__.__name__ == 'Predictor' and P.get_mirrored_patch_crops(batch['patch_crop_coords'], batch['original_img_shape']) == \
-        ref_predictor.get_mirrored_patch_crops(batch['patch_crop_coords'], batch['original_img_shape'])
+    assert a['seg_preds'].shape == (1, 4, 48, 48, 24) and digest(a['seg_preds']) == b['seg_preds']
+    assert ours.__class__.__name__ == 'Predictor' and \
+        plain(P.get_mirrored_patch_crops(batch['patch_crop_coords'], batch['original_img_shape'])) == b['mirrored_crops']
 
     # the temporal-ensembling loop with stand-in checkpoints (the reference consolidates in a 6-process pool; here: in-process)
     class Net(StandInNet):
